@@ -12,6 +12,8 @@ refinement), step lengths, iterate update.
 
   python bench.py --gpus N --steps K --warmup W          our CUDA path
   python bench.py --impl reference ...                   reference algorithm on the host CPU
+  python bench.py ... --dump-outputs DIR                 also write the solution of the last timed solve as DIR/*.npy
+                                                         (--impl reference: the iterate of its bounded CPU solve)
 
 `value`  : K real iterations (after W untimed warm-up iterations) timed with CUDA
            events on the solver's stream, problem resident in HBM.
@@ -35,6 +37,20 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+DUMP_CAP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays, cap=DUMP_CAP_BYTES):
+    """Write each array as out_dir/<name>.npy in float64, so that two builds can be compared output for output on the
+    same seeded inputs.  Past `cap` bytes in all, every array is cut to a fixed, seeded sample of its entries."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64).reshape(-1) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > cap:
+            keep = a.size * (cap - 4096 * len(arrays)) // total        # 4 KB per file leaves room for the .npy header
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_workload(name, rank):
@@ -327,6 +343,8 @@ def run_ours(args, rank, world):
             "cpu_baseline": cpu,
         }
     solver.close()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: r[k] for k in ("x", "z", "s")})
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -410,6 +428,8 @@ def run_reference(args, rank, world):
     # bounded sample: the whole arm has to end within a few minutes; an iteration of the port costs ~12 s on C4
     cap = {"c4": 6, "c5": 4}.get(args.workload, W + K)
     ipm, r, t_setup, t_total, order = cpu_solve(pr, args.workload, min(W + K, cap))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: r[k] for k in ("x", "z", "s")})
     i = r["info"]
     iters = r["iterations"]
     value = iters / i.solve_time
@@ -446,6 +466,10 @@ def main():
                     help="with --gpus N > 1: N independent problems (weak scaling) instead of ONE problem split over the N GPUs")
     ap.add_argument("--no-process-warmup", action="store_true",
                     help="skip the tiny warm-up problem (for ncu launch lists: keeps the capture on the workload)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write x, z and s of the last timed solve as DIR/<name>.npy (float64); "
+                         "with --impl reference: the iterate where its bounded solve stopped (min(W+K, 6) iterations "
+                         "on c4, min(W+K, 4) on c5), which is not converged and so not comparable with the CUDA arm's")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -471,4 +495,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the benchmark writes nothing into the source tree (it may be read-only)
     main()

@@ -24,44 +24,43 @@ def build_flags():
     return _build
 
 
-def _native_path():
+def _native_lib():
     """ORACLE_NATIVE=1 (set by bench.py's CPU legs): compile the port for THIS host, `gcc -O3 -march=native`
-    (BASELINE.md section 3), into oracle/_native/ (git-ignored).  The portable library stays the fallback: a library
-    built with -march=native on one machine may not run on another, so it is never shipped."""
-    import subprocess
+    (BASELINE.md section 3), into a new private directory (mkdtemp: owned by this user, mode 0700, unpredictable
+    name), load it and delete the directory again.  Nothing is written into the source tree, which may be read-only,
+    nothing is left behind, and no library that another user could have placed is ever loaded.  The portable library
+    stays the fallback: a library built with -march=native on one machine may not run on another, so it is never
+    shipped."""
     import glob
+    import shutil
+    import subprocess
+    import tempfile
     if os.environ.get("ORACLE_NATIVE", "0") != "1":
         return None
-    out_dir = os.path.join(_HERE, "_native")
-    out = os.path.join(out_dir, "liboracle_native.so")
     srcs = sorted(glob.glob(os.path.join(_HERE, "*.c")))
-    deps = srcs + sorted(glob.glob(os.path.join(_HERE, "*.h")))
+    tmp = tempfile.mkdtemp(prefix="clarabel_b200_oracle_")
     try:
-        stamp = os.path.join(out_dir, "host.txt")
-        host = open("/proc/cpuinfo").read().split("model name", 2)[1].split("\n")[0] if os.path.exists("/proc/cpuinfo") else ""
-        fresh = (os.path.exists(out) and os.path.exists(stamp) and open(stamp).read() == host
-                 and all(os.path.getmtime(out) >= os.path.getmtime(d) for d in deps))
-        if not fresh:
-            os.makedirs(out_dir, exist_ok=True)
-            subprocess.check_call(["gcc", "-O3", "-march=native", "-fPIC", "-shared", "-o", out] + srcs + ["-lm"],
-                                  stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, timeout=300)
-            open(stamp, "w").write(host)
-        return out
+        out = os.path.join(tmp, "liboracle_native.so")
+        subprocess.check_call(["gcc", "-O3", "-march=native", "-fPIC", "-shared", "-o", out] + srcs + ["-lm"],
+                              stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, timeout=300)
+        return C.CDLL(out)          # the mapping outlives the file
     except Exception:
         return None
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)
 
 
 def lib():
     global _lib, _build
     if _lib is None:
         path = os.path.join(_HERE, "liboracle.so")
-        native = _native_path()
-        if native is not None:
-            path = native
-            _build = "-O3 -march=native, compiled on this host (oracle/_native/)"
-        if not os.path.exists(path):
+        L = _native_lib()
+        if L is not None:
+            _build = "-O3 -march=native, compiled on this host"
+        elif not os.path.exists(path):
             raise RuntimeError("oracle/liboracle.so missing: run `make` (or __graft_entry__.build())")
-        L = C.CDLL(path)
+        else:
+            L = C.CDLL(path)
         vp = C.c_void_p
         L.oq_new.argtypes = [C.POINTER(vp), C.c_int64, C.c_int64, i64p, i64p, f64p, i64p, i8p,
                              C.c_int, C.c_int, C.c_double, C.c_double]

@@ -1,5 +1,5 @@
-"""The reference's JSON problem format (default/json.rs:11-95): round trip through clarabel.rs_b200/jsonio.py and,
-when the reference tree is present (this container, not the GPU box), its own examples/data/hs35.json.  CPU only."""
+"""The reference's JSON problem format (default/json.rs:11-95): round trip through clarabel.rs_b200/jsonio.py and its
+own examples/data/hs35.json, stored verbatim as tests/golden/reference_data/hs35.json.  CPU only."""
 import importlib.util
 import json
 import os
@@ -45,9 +45,8 @@ def test_rejects_unknown_cones(tmp_path):
             jsonio.load_problem(p)
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/examples/data/hs35.json"), reason="reference tree not present")
 def test_reference_data_file_hs35():
-    d = jsonio.load_problem("/root/reference/examples/data/hs35.json")
+    d = jsonio.load_problem(os.path.join(os.path.dirname(__file__), "golden", "reference_data", "hs35.json"))
     P, q, A, b, cones = rp.hs35()
     assert (d["P"] != P).nnz == 0 and (d["A"] != A).nnz == 0 and list(d["q"]) == q and list(d["b"]) == b
     assert d["cones"] == cones
